@@ -5,6 +5,7 @@ independent 64 KB blocks (tests/datagen P50), per GPU count, against the HBM roo
     python bench.py [--gpus N --steps K --warmup W]          our CUDA path
     python bench.py --impl reference [...]                    the reference's CPU implementation
     torchrun --nproc-per-node N bench.py --gpus N ...         one rank per GPU (weak scaling)
+    python bench.py [...] --dump-outputs DIR                  + what the last timed step decoded, as DIR/*.npy
 
 One "step" = one pass of the hot path (scan + expand kernels) over this rank's whole batch
 (default 4 GiB = 65 536 blocks per GPU).  Inputs are device resident for `value`; `e2e` runs the
@@ -52,7 +53,42 @@ def parse_args():
                     help="N > 1: 'nccl' = grouped NCCL send/recv per chunk, 'peer' = copy-engine pushes into the peers' frames (CUDA IPC)")
     ap.add_argument("--reserve-sms", type=int, default=0,
                     help="N > 1: SMs the persistent decode kernels leave to the concurrent exchange kernels (LZ4B200_RESERVE_SMS)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step decoded to DIR/*.npy (a fixed, seeded sample)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+# --------------------------------------------------------------------------------------------
+# --dump-outputs: the decoded frame of the last timed step, so that two builds can be compared output for output
+# --------------------------------------------------------------------------------------------
+DUMP_DECODED_BYTES = 4 << 20        # decoded bytes sampled into decoded_blocks.npy (16 MiB as float32)
+DUMP_MAX_SIZES = 1 << 21            # per-block return values written in full up to this many blocks, else a sample
+
+
+def dump_outputs(dirname, n_blocks, block_rows, sizes):
+    """Write decoded_blocks.npy (float32: the bytes of whole blocks picked with a fixed seed, at most
+    DUMP_DECODED_BYTES in all), decoded_block_ids.npy (their indices) and decoded_sizes.npy (the return value of
+    every block; beyond DUMP_MAX_SIZES blocks a seeded sample, with decoded_sizes_ids.npy).  block_rows(ids) gives
+    the decoded bytes of blocks `ids` as a (len(ids), >= width) uint8 array; sizes is the int array of all returns.
+    The same arguments give the same blocks, and the dump stays below 64 MB whatever the workload size."""
+    os.makedirs(dirname, exist_ok=True)
+
+    def pick(k):
+        if n_blocks <= k:
+            return np.arange(n_blocks)
+        return np.sort(np.random.default_rng(0).choice(n_blocks, k, replace=False))
+
+    width = min(BLOCK, DUMP_DECODED_BYTES)
+    ids = pick(max(1, DUMP_DECODED_BYTES // BLOCK))
+    np.save(os.path.join(dirname, "decoded_block_ids.npy"), ids.astype(np.float64))
+    np.save(os.path.join(dirname, "decoded_blocks.npy"), np.asarray(block_rows(ids))[:, :width].astype(np.float32))
+    ids = pick(DUMP_MAX_SIZES)
+    if len(ids) < n_blocks:
+        np.save(os.path.join(dirname, "decoded_sizes_ids.npy"), ids.astype(np.float64))
+    np.save(os.path.join(dirname, "decoded_sizes.npy"), np.asarray(sizes)[ids].astype(np.float64))
 
 
 # --------------------------------------------------------------------------------------------
@@ -177,6 +213,8 @@ def run_reference(args):
         assert t > 0 and (rets == BLOCK).all()
         times.append(t)
     assert (out == data).all(), "reference round trip mismatch"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n_blocks, lambda ids: out.reshape(n_blocks, BLOCK)[ids], rets)
     med, best, mean = float(np.median(times)), min(times), sum(times) / len(times)
     nbytes = n_blocks * BLOCK
     value = nbytes / med / GB
@@ -415,6 +453,16 @@ def run_ours(args):
         elapsed_ms = float(t.max().item())
     value = world * total * K / (elapsed_ms * 1e-3) / GB
     clocks = sampler.summary(t_wall0, t_wall1)
+    if args.dump_outputs:                       # before the phase timing below decodes again into the same frame
+        all_rets = rets
+        if world > 1:
+            all_rets = torch.empty(world * n_blocks, dtype=torch.int32, device=device)
+            dist.all_gather_into_tensor(all_rets, rets)
+        if rank == 0:
+            width = min(BLOCK, DUMP_DECODED_BYTES)
+            dump_outputs(args.dump_outputs, world * n_blocks,
+                         lambda ids: full.view(-1, BLOCK)[torch.from_numpy(ids).to(device), :width].cpu().numpy(),
+                         all_rets.cpu().numpy())
 
     # ---- the two kernels of the decode, timed separately (same launches, events between the phases) ----
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(K)]

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Generate tests/golden/*.json from the COMPILED REFERENCE (oracle/_ref/libref_lz4.so).
 
-Run in the build container, where /root/reference exists:
+Run where the reference sources exist (oracle/Makefile, REF=<path>):
     make -C oracle ref && python tests/golden/make_golden.py
 The reference ships no golden compressed vectors for the block codec (SURVEY.md section 8c), so
 these fixtures are outputs of the reference itself: every `ret`, `out` and digest below was
@@ -148,6 +148,40 @@ def main():
     with open(os.path.join(HERE, "p50_seed0_64k.lz4block"), "wb") as f:
         f.write(c)
     print("decode cases", len(decode), "compress cases", len(comp), "datagen rows", len(dg), "block", len(c), "frames", len(frames))
+    reference_answers(ref)
+
+
+def reference_answers(ref):
+    """tests/golden/ref_answers.json: the reference's answers to the seeded cases of tests/ref_answers.py"""
+    import re
+    import subprocess
+    import tempfile
+    sys.path.insert(0, os.path.dirname(HERE))
+    import ref_answers as ra
+
+    ans = {"source": "lz4 v1.10.0: lib/lz4.c, lib/lz4frame.c, tests/datagen.c (gcc -O3 x86-64) and the programs/ "
+                     "command-line tool, run on the cases of tests/ref_answers.py",
+           "datagen": ra.datagen_records(ref),
+           "compress": ra.compress_records(ref, ref),
+           "noisy": ra.noisy_records(ref, ref),
+           "frames": [ra.frame_record(ref.compress_frame(d, bsid, level, csf)) for d, bsid, level, csf in ra.frame_cases(ref)],
+           "fuzz": {str(s): ra.fuzz_records(ref, ref, s) for s in ra.FUZZ_SEEDS}}
+    cli = os.path.join(ROOT, "oracle", "_ref", "lz4")
+    bench = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        paths = ra.write_bench_files(ref, tmp)
+        for args, idx in ra.BENCH_COMMANDS:
+            sub = [paths[i] for i in idx]
+            r = subprocess.run([cli] + args + sub, capture_output=True, text=True, timeout=120)
+            text = (r.stdout + r.stderr).replace("\r", "\n")
+            m = re.findall(r":\s*(\d+) ->\s*(\d+) \(([\d.]+)\),\s*[\d.]+ MB/s,\s*[\d.]+ MB/s", text)
+            assert r.returncode == 0 and m, text
+            bench[ra.bench_key(args, sub)] = [int(m[-1][0]), int(m[-1][1]), m[-1][2]]
+    ans["lz4_bench"] = bench
+    with open(ra.GOLDEN, "w") as f:
+        json.dump(ans, f, separators=(",", ":"))
+        f.write("\n")
+    print("reference answers:", {k: len(v) for k, v in ans.items() if k != "source"})
 
 
 if __name__ == "__main__":

@@ -1,22 +1,20 @@
 """lz4_b200.lz4bench (SURVEY.md section 8 f-2): the `lz4 -b` harness.
 
 CPU part: the codec-agnostic harness is driven by an oracle-backed codec (test infrastructure) and
-its block split / level rule / sizes / ratio / result lines are compared with the REFERENCE TOOL
-`lz4 -b# -i0` (oracle/_ref/lz4, compiled from programs/*.c) on the same files.
+its block split / level rule / sizes / ratio / result lines are compared with what the REFERENCE TOOL
+`lz4 -b# -i0` (programs/*.c) printed for the same files (tests/golden/ref_answers.json).
 GPU part: the same comparison for the product codec (GpuCodec).
 """
 import os
 import re
-import subprocess
 import time
 
 import numpy as np
 import pytest
 
+import ref_answers as ra
 from lz4_b200 import lz4bench
-from oracle.pyoracle import Oracle, Reference, have_reference
-
-REF_CLI = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "lz4")
+from oracle.pyoracle import Oracle
 
 
 class OracleCodec(lz4bench.Codec):
@@ -69,26 +67,13 @@ class OracleCodec(lz4bench.Codec):
 
 @pytest.fixture(scope="module")
 def files(tmp_path_factory):
-    gen = Reference() if have_reference() else Oracle()
-    d = tmp_path_factory.mktemp("benchfiles")
-    specs = [("p50.bin", 300000, 0.5, 0), ("p90.bin", 70001, 0.9, 1), ("tiny.bin", 40, 0.5, 2), ("p20.bin", 131072, 0.2, 3)]
-    paths = []
-    for name, n, p, seed in specs:
-        path = d / name
-        path.write_bytes(bytes(gen.datagen(n, p, seed)))
-        paths.append(str(path))
-    return paths
+    return ra.write_bench_files(Oracle(), tmp_path_factory.mktemp("benchfiles"))
 
 
-def ref_bench(paths, level_flag, block_flag=None):
-    """Run the reference tool: lz4 -b# -i0 [-B#] files -> (srcSize, cSize, ratio text)."""
-    cmd = [REF_CLI, level_flag, "-i0"] + ([block_flag] if block_flag else []) + list(paths)
-    out = subprocess.run(cmd, capture_output=True, text=True, timeout=120)
-    text = (out.stdout + out.stderr).replace("\r", "\n")
-    m = re.findall(r":\s*(\d+) ->\s*(\d+) \(([\d.]+)\),\s*[\d.]+ MB/s,\s*[\d.]+ MB/s", text)
-    assert m, text
-    src, csz, ratio = m[-1]
-    return int(src), int(csz), ratio
+def ref_bench(args, paths):
+    """What the reference tool printed for `lz4 <args> <files>`: (srcSize, cSize, ratio text)."""
+    src, csz, ratio = ra.load()["lz4_bench"][ra.bench_key(args, paths)]
+    return src, csz, ratio
 
 
 def test_split_blocks_never_straddle_files():
@@ -127,7 +112,6 @@ def test_fastest_pass_rule_and_loop_sizing():
     assert calls == [1] and passes == 1 and fastest == 7
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="reference CLI not built (make -C oracle ref)")
 @pytest.mark.parametrize("level_flag,level,block_flag,block", [
     ("-b1", 1, "-B4", 65536), ("-b1", 1, None, 0), ("-b0", 0, "-B5", 262144), ("-b1", 1, "-B1000", 1000),
 ])
@@ -137,7 +121,7 @@ def test_harness_matches_reference_tool(files, level_flag, level, block_flag, bl
         sizes = [os.path.getsize(p) for p in subset]
         name = os.path.basename(subset[0]) if len(subset) == 1 else " %u files" % len(subset)
         res = lz4bench.bench_mem(OracleCodec(), src, sizes, name, level, block, nb_seconds=0)
-        rsrc, rcsz, rratio = ref_bench(subset, level_flag, block_flag)
+        rsrc, rcsz, rratio = ref_bench([level_flag, "-i0"] + ([block_flag] if block_flag else []), subset)
         assert res.error == 0
         assert (res.src_size, res.c_size) == (rsrc, rcsz)
         assert "%5.3f" % res.ratio == rratio
@@ -146,14 +130,11 @@ def test_harness_matches_reference_tool(files, level_flag, level, block_flag, bl
         assert res.quiet_line().startswith("-%-3i%11i (%s)" % (level, rcsz, rratio))
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="reference CLI not built (make -C oracle ref)")
 def test_fast_levels_match_reference_tool(files):
     src = open(files[0], "rb").read()
     for fast in (1, 3, 9):
         res = lz4bench.bench_mem(OracleCodec(), src, [len(src)], "p50.bin", -fast, 65536, nb_seconds=0)
-        out = subprocess.run([REF_CLI, "--fast=%d" % fast, "-b", "-i0", "-B4", files[0]], capture_output=True, text=True, timeout=60)
-        m = re.findall(r":\s*(\d+) ->\s*(\d+) \(", (out.stdout + out.stderr).replace("\r", "\n"))
-        assert m and (res.src_size, res.c_size) == (int(m[-1][0]), int(m[-1][1]))
+        assert (res.src_size, res.c_size) == ref_bench(["--fast=%d" % fast, "-b", "-i0", "-B4"], files[:1])[:2]
 
 
 def test_verify_reports_corruption(files, capsys):
@@ -172,7 +153,6 @@ def test_cli_refuses_hc_and_needs_files():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not os.path.exists(REF_CLI), reason="reference CLI not built")
 def test_gpu_codec_matches_reference_tool(files):
     codec = lz4bench.GpuCodec()
     for subset, level, level_args, block_flag, block in ((files[:1], 1, ["-b1"], "-B4", 65536),
@@ -182,9 +162,6 @@ def test_gpu_codec_matches_reference_tool(files):
         src = b"".join(open(p, "rb").read() for p in subset)
         sizes = [os.path.getsize(p) for p in subset]
         res = lz4bench.bench_mem(codec, src, sizes, "x", level, block, nb_seconds=0)
-        out = subprocess.run([REF_CLI] + level_args + ["-i0"] + ([block_flag] if block_flag else []) + list(subset),
-                             capture_output=True, text=True, timeout=120)
-        m = re.findall(r":\s*(\d+) ->\s*(\d+) \(", (out.stdout + out.stderr).replace("\r", "\n"))
         assert res.error == 0
-        assert m and (res.src_size, res.c_size) == (int(m[-1][0]), int(m[-1][1]))
+        assert (res.src_size, res.c_size) == ref_bench(level_args + ["-i0"] + ([block_flag] if block_flag else []), subset)[:2]
         assert res.c_ns > 0 and res.d_ns > 0
